@@ -2,6 +2,7 @@
 """bench.py -- BASELINE.json's headline metric on B200, plus one short leg per other BASELINE config.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c2null|c1|c4|c5]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Headline (BASELINE.json configs[1] / [2], SURVEY.md 8(d) "C2/C3"): a 1 B-row table of 8 int8 columns in 32
@@ -23,6 +24,8 @@ over NVLink at N > 1) and the compaction of the result rows.
   --impl reference  the CPU restatement of the reference's path (oracle/, one pinned thread per shard, shards
           written by the oracle's own row-at-a-time writer: nothing of citus_b200 is loaded) on the box's host
           cores -- NOT PostgreSQL/Citus, which cannot be built here
+  --dump-outputs DIR  after the timed steps of the headline, the result rows of its last step as DIR/<name>.npy
+          (see dump_c2_result); the inputs are seeded, so two builds can be compared output for output
 """
 from __future__ import annotations
 
@@ -77,7 +80,13 @@ def parse():
     p.add_argument("--no-numa-bind", action="store_true", help="do not pin the rank to the CPUs of its GPU's NUMA node")
     p.add_argument("--leg-steps", type=int, default=5)
     p.add_argument("--leg-timeout", type=float, default=240.0, help="deadline in seconds for each extra leg")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", help="write the result rows of the headline's last timed step as DIR/<name>.npy")
+    a = p.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        p.error("--steps must be at least 1 and --warmup at least 0")
+    if a.dump_outputs and (a.impl != "ours" or a.workload != "c2"):
+        p.error("--dump-outputs writes the headline's result: it needs --impl ours and --workload c2")
+    return a
 
 
 class ClockSampler(threading.Thread):
@@ -255,6 +264,28 @@ def dense_from_gpu(fetch, nkeys, sum_agg=0, count_agg=1):
     Cn[k] = fetch["count"][:n, count_agg]
     Nn[k] = fetch["count"][:n, sum_agg]
     return S, Cn, Nn
+
+
+def dump_c2_result(out_dir, fetch, sum_agg=0, count_agg=1):
+    """the rows of SELECT key, sum(v), count(*) ... GROUP BY key as the caller receives them (cg_partial_fetch), ordered
+    by key with the NULL group last, one .npy per column: key, key_is_null, sum_v (NaN where sum(v) is NULL),
+    count_star.  float64 holds every key, count and sum exactly (|value| < 2^53 is checked); 28 bytes per group, 28 MB
+    for the headline's 1 M groups."""
+    n = fetch["n"]
+    kn = fetch["key_nulls"][:n] != 0
+    keys = np.where(kn, 0, fetch["keys"][:n])
+    lo = fetch["sum_lo"][:n, sum_agg].view(np.int64)
+    assert np.array_equal(fetch["sum_hi"][:n, sum_agg], lo >> 63), "sum does not fit int64"
+    exact = 1 << 53
+    assert np.abs(keys).max(initial=0) < exact and np.abs(lo).max(initial=0) < exact, "not exact in float64"
+    order = np.lexsort((keys, kn))
+    cols = {"key": keys.astype(np.float64), "key_is_null": kn.astype(np.float32),
+            "sum_v": np.where(fetch["count"][:n, sum_agg] > 0, lo.astype(np.float64), np.nan),
+            "count_star": fetch["count"][:n, count_agg].astype(np.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in cols.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a[order])
+    log(f"wrote {n} result rows ({sum(a.nbytes for a in cols.values()) / 1e6:.1f} MB) to {out_dir}")
 
 
 def reduce_host_arrays(arrays, world):
@@ -625,6 +656,8 @@ def run_c2(env, args, nulls=False, headline=True):
                                 "NVLink into the root's window; flag barriers in peer memory") if cgd.peer_window() else "ncclReduce"
     ms, clocks, all_launches, nscan, ktotal, last = env.timed(step, steps, warmup)
     ngroups = last[0] if last else 0
+    if headline and args.dump_outputs and rank == 0:
+        dump_c2_result(args.dump_outputs, partial.fetch())      # the partial still holds the last timed step's result
     value = total_rows / (ms / 1e3)
     if world > 1 and headline:
         # where a step's time goes on this rank (events between the phases; outside the timed loop)
@@ -673,11 +706,24 @@ def run_c2(env, args, nulls=False, headline=True):
     e2e = None
     if headline and not args.no_e2e:
         t0 = time.time()
-        if not args.pageable:
-            for s in my_shards:               # pin the page images once
-                rels[s].register()
+        pinned, refused = not args.pageable, None
+        if pinned:
+            try:
+                for s in my_shards:           # pin the page images once
+                    rels[s].register()
+            except capi.CitusGpuError as e:
+                refused = f"rank {rank}: {e}"
+            if env.sum_over_ranks([refused is not None])[0]:
+                # the OS would not pin every image (an unprivileged process can be refused): every rank times the
+                # pageable path instead, and the line says so
+                refused = refused or "refused on another rank"
+                for s in my_shards:
+                    rels[s].unregister()
+                pinned = False
+                log(f"rank {rank}: page images not pinned ({refused}); e2e uses pageable pages")
         reg_s = time.time() - t0
-        log(f"rank {rank}: registered {len(my_shards)} page images in {reg_s:.1f}s")
+        if pinned:
+            log(f"rank {rank}: registered {len(my_shards)} page images in {reg_s:.1f}s")
         partial.reset()
         h2d = 0
         for s in my_shards:                   # instrumented warm-up pass: bytes moved
@@ -701,13 +747,15 @@ def run_c2(env, args, nulls=False, headline=True):
         h2d = env.sum_over_ranks([h2d])[0]
         e2e = {"value": total_rows / (ems / 1e3), "unit": "rows/s", "h2d_bytes_per_step": int(h2d),
                "d2h_bytes_per_step": int(d2h[0]), "ms_per_step": ems, "steps": max(args.e2e_steps, 5),
-               "host_buffers": "pageable pages -> host de-frame into pinned blocks -> cudaMemcpyAsync" if args.pageable else
+               "host_buffers": "pageable pages -> host de-frame into pinned blocks -> cudaMemcpyAsync" if not pinned else
                                "pinned (cudaHostRegister) page images -> 1-D DMA of whole pages -> GPU drops page headers + realigns",
-               "assumption": None if args.pageable else
+               "assumption": None if not pinned else
                              f"the page images are pinned ONCE, outside the timed region ({reg_s:.1f} s for this rank's {len(my_shards)} shards "
                              f"here): what registering the shared_buffers segment at postmaster start would do; --pageable times the "
                              f"path that needs no registration",
                "api": "cg_scan_relation + cg_comm_combine + cg_partial_fetch", "numa_node": env.numa_node}
+        if refused:
+            e2e["pinning_refused"] = refused
         for s in my_shards:
             rels[s].unregister()
 

@@ -1136,7 +1136,15 @@ extern "C" int cg_relation_register(const CgRelation *rel)
 {
 	if (!cg_ctx()) return CG_EINVAL;
 	if (!rel || !rel->pages || rel->nblocks == 0) return cg_set_error(CG_EINVAL, "empty relation");
-	CG_CUDA(cudaHostRegister((void *) rel->pages, (size_t) rel->nblocks * CG_BLCKSZ, cudaHostRegisterDefault));
+	size_t bytes = (size_t) rel->nblocks * CG_BLCKSZ;
+	cudaError_t e = cudaHostRegister((void *) rel->pages, bytes, cudaHostRegisterDefault);
+	if (e != cudaSuccess)
+	{
+		/* the OS may refuse to pin the range (an unprivileged process can be refused): the caller can go on
+		 * with pageable pages, so the refusal must not linger as the thread's last CUDA error */
+		cudaGetLastError();
+		return cg_set_error(CG_ECUDA, "cudaHostRegister of %zu bytes failed: %s", bytes, cudaGetErrorString(e));
+	}
 	return CG_OK;
 }
 

@@ -291,7 +291,8 @@ int cg_scan_shard(const CgShard *shard, const CgScanDesc *desc, CgPartial *into,
  * pinned memory (cg_relation_register, or a shared_buffers segment registered once at
  * startup) are sent by the copy engine itself as runs of whole pages (1-D copies);
  * the GPU drops the page headers and re-aligns the chunk buffers. */
-int cg_relation_register(const CgRelation *rel);      /* cudaHostRegister of the page image */
+int cg_relation_register(const CgRelation *rel);      /* cudaHostRegister of the page image; CG_ECUDA if the OS
+                                                        * refuses to pin it (the pages stay usable, as pageable) */
 int cg_relation_unregister(const CgRelation *rel);
 int cg_scan_relation(const CgRelation *rel, const CgScanDesc *desc, CgPartial *into, CgScanStats *stats);
 

@@ -42,10 +42,17 @@ def test_no_oracle_in_product():
 
 
 def test_calls_fail_loudly_without_init(cg):
-    from citus_b200 import capi
-    d = cg.make_desc(aggs=[cg.count_star()])
-    with pytest.raises(capi.CitusGpuError):
-        cg.GpuColumnarAgg(d, [(8, 0)])
+    # in a process of its own: the GPU tests of the same session may already have called cg_init in this one
+    import subprocess
+    import sys
+    code = ("import sys; sys.path.insert(0, sys.argv[1])\n"
+            "from citus_b200 import capi, columnar as cg\n"
+            "try:\n"
+            "    cg.GpuColumnarAgg(cg.make_desc(aggs=[cg.count_star()]), [(8, 0)])\n"
+            "except capi.CitusGpuError as e:\n"
+            "    print('refused:', e)\n")
+    r = subprocess.run([sys.executable, "-c", code, ROOT], capture_output=True, text=True, timeout=300)
+    assert r.returncode == 0 and r.stdout.startswith("refused:") and "cg_init" in r.stdout, r.stdout + r.stderr
 
 
 def _same_image(rel, t):

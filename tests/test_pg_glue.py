@@ -46,11 +46,9 @@ def test_c_driver_builds_and_fails_loudly_without_a_gpu(tmp_path):
     build.build()
     orc.build()
     exe = _build_driver(tmp_path)
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("covered by the gpu test")
+    # where a GPU is present, the driver is shown none (CUDA_VISIBLE_DEVICES empty)
     r = subprocess.run([exe, os.path.join(ROOT, "citus_b200", "lib", "libcitus_gpu.so"), os.path.join(ROOT, "oracle", "liboracle.so")],
-                       capture_output=True, text=True)
+                       capture_output=True, text=True, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
     assert r.returncode == 1 and "cg_init" in r.stderr            # no device: an error, never a CPU fallback
 
 
